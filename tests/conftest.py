@@ -14,8 +14,18 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
+    import json
     import numpy as np
-    return np.load(os.path.join(ROOT, "tests", "golden", "unet_sampler_golden.npz"))
+    with np.load(os.path.join(ROOT, "tests", "golden", "unet_sampler_golden.npz")) as z:
+        g = dict(z)
+    # the tiny-UNet inputs are not stored: tests/golden/make_golden.py drew them first from default_rng(7), so they are
+    # regenerated bit for bit, as the weights are from their seeds
+    rng = np.random.default_rng(7)
+    for tag in ("tiny", "tiny_cond", "tiny_sr"):
+        cfg = json.loads(bytes(g[f"{tag}_cfg"]).decode())
+        S = cfg["image_size"]
+        g[f"{tag}_x"] = rng.standard_normal((len(g[f"{tag}_t"]), cfg["in_channels"], S, S)).astype(np.float32)
+    return g
 
 
 @pytest.fixture(scope="session", autouse=True)
